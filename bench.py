@@ -2,6 +2,7 @@
 """bench.py -- the SdfKit hot path on B200: SdfExpr.ToSdf() -> Voxels sampling -> MarchingCubes meshing.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--grid N] [--scene readme|csg50|sphere]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one grid of the README RepeatXY scene (BASELINE.json): sample every
 voxel (distance + colour, clip to bounds) into HBM, then mesh it (classify -> scan -> compact -> emit).  The SDF
@@ -20,6 +21,9 @@ Outside the timed regions the line also carries
   configs (N = 1)       BASELINE configs 3 (CSG-50 1024^3, FP32-bound) and 5 (ToImage 1920x1080, Perf/Program.cs protocol)
                         with their own FP32 rooflines and CPU baselines, and the Voxels.Values/Colors export rate.
 --impl reference times the CPU restatement of the reference (the oracle) on a bounded sample of the workload.
+--dump-outputs DIR writes the mesh of the last timed step as DIR/<name>.npy, so that two builds can be compared output for
+output (the inputs are the same in every run: an analytic SDF on a fixed grid).
+bench.py writes nothing into the tree it runs from, which may be read-only: the oracle compiles into a temporary directory.
 """
 import argparse
 import hashlib
@@ -31,6 +35,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True          # no __pycache__ in the tree for modules build() did not import
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -73,6 +78,31 @@ def mesh_sha(m):
     import numpy as np
     return {k: hashlib.sha256(np.ascontiguousarray(getattr(m, a)).tobytes()).hexdigest()
             for k, a in (("vertices", "Vertices"), ("colors", "Colors"), ("normals", "Normals"), ("triangles", "Triangles"))}
+
+
+DUMP_ROWS = 1 << 19        # rows kept of each mesh array: ~40 MB of .npy files in all
+
+
+def dump_outputs(job, dev, out_dir):
+    """The mesh the last timed step left on the device, i.e. what a caller of the step receives, as .npy files: vertices,
+    colors, normals (float32 [rows, 3]) and triangles (float64 [rows, 3]; the int32 vertex ids are exact in float64).
+    A mesh with more than DUMP_ROWS vertices (triangles) is represented by the same seeded sample of rows in every run;
+    counts.npy holds the full (vertices, triangles) counts, vertex_rows.npy / triangle_rows.npy the rows kept."""
+    import numpy as np
+    import torch
+    from sdfkit_b200 import dist as skd
+    parts = [skd.mesh_device_tensors(s.mesh, dev) for s in job.slabs if s.mesh is not None]
+    v, c, nrm, t = (torch.cat([p[a] for p in parts]) for a in range(4))
+
+    def rows(n, seed):
+        return np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(seed).choice(n, DUMP_ROWS, replace=False))
+    vr, tr = rows(len(v), 1), rows(len(t), 2)
+    vi, ti = torch.as_tensor(vr, device=dev), torch.as_tensor(tr, device=dev)
+    out = {"counts": np.float64([len(v), len(t)]), "vertex_rows": vr.astype(np.float64), "triangle_rows": tr.astype(np.float64),
+           "vertices": v[vi], "colors": c[vi], "normals": nrm[vi], "triangles": t[ti].double()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy() if torch.is_tensor(a) else a)
 
 
 def golden_digest(scene, n):
@@ -503,6 +533,8 @@ def run_ours(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the SdfKit GPU path has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the mesh of a one-process run: use it with --gpus 1")
     torch.cuda.set_device(local)
     import torch.distributed as dist
     host_group = None
@@ -738,6 +770,8 @@ def run_ours(args):
     parity = None
     if world > 1 and not args.no_parity:
         parity = parity_check(sk, skd, dist, torch, ctx, sdf, job, last_allc, last_offs, expr, mn, mx, n, rank, world, dev, args.scene)
+    if args.dump_outputs:
+        dump_outputs(job, dev, args.dump_outputs)
     job.close()
 
     # ---- rank 0 alone: strong scaling through the multi-GPU C ABI, BASELINE configs 3 / 5, export, CPU baseline
@@ -929,7 +963,12 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the N-rank parity block")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling block (multi-GPU context of the C ABI)")
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE config 3 / 5 / export sub-records (N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the mesh of the last one as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computed")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -8,16 +8,19 @@ batched `Sdf` delegate (SdfKit/Sdf.cs:8):
     opaque `fn(points[n,3]) -> out[n,4]`, wrapped as a C callback.  This is how the reference's own
     tests (opaque C# lambdas such as Sdfs.Sphere) are restated.
 """
+import atexit
 import ctypes as C
 import hashlib
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _PRELUDE = os.path.join(os.path.dirname(_HERE), "sdfkit_b200", "csrc", "sdfk_prelude.h")
-_CACHE = os.path.join(_HERE, "_sdfcache")
+_CACHE = None       # compiled SDFs: a temporary directory of this process (the source tree may be read-only)
 _LIB = None
 
 SDF_FN = C.CFUNCTYPE(None, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int)
@@ -96,7 +99,10 @@ def compile_sdf(body):
     body = getattr(body, "body", body)
     src = _WRAPPER % {"prelude": _PRELUDE, "body": body}
     key = hashlib.sha256(src.encode()).hexdigest()[:24]
-    os.makedirs(_CACHE, exist_ok=True)
+    global _CACHE
+    if _CACHE is None:
+        _CACHE = tempfile.mkdtemp(prefix="sdfk_oracle_")
+        atexit.register(shutil.rmtree, _CACHE, True)
     so = os.path.join(_CACHE, "sdf_%s.so" % key)
     if not os.path.exists(so):
         cpp = os.path.join(_CACHE, "sdf_%s.cpp" % key)

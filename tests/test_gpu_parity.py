@@ -728,3 +728,31 @@ def test_store_bandwidth_probe(sk):
     with pytest.raises(N.SdfkError):
         ctx.store_bandwidth(1024, 1)            # less than one 16 KiB chunk
     ctx.close()
+
+
+def test_bench_dump_outputs_is_the_mesh_of_the_timed_step(sk, tmp_path):
+    """`bench.py --dump-outputs DIR` writes the mesh of the last timed step.  On a grid small enough to keep every row, that
+    is the mesh Sdf.ToMesh makes of the same grid, bit for bit; the JSON line reports the --steps asked for."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from sdfkit_b200 import scenes
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n = 96
+    cmd = [sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "0", "--grid", str(n), "--no-cpu", "--no-configs",
+           "--no-strong", "--no-e2e", "--no-fused", "--dump-outputs", str(tmp_path)]
+    r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=root)
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == 2
+    expr, mn, mx = scenes.readme_scene()
+    m = expr.ToSdf().ToMesh(mn, mx, n, n, n)
+    d = {k: np.load(tmp_path / (k + ".npy")) for k in ("counts", "vertex_rows", "triangle_rows", "vertices", "colors", "normals", "triangles")}
+    nv, nt = len(m.Vertices), len(m.Triangles) // 3
+    assert d["counts"].tolist() == [nv, nt] == [line["vertices"], line["triangles"]]
+    assert np.array_equal(d["vertex_rows"], np.arange(nv)) and np.array_equal(d["triangle_rows"], np.arange(nt))
+    for k in ("vertices", "colors", "normals"):
+        assert d[k].dtype == np.float32
+        assert_bits_equal(d[k], getattr(m, k.capitalize()), k)
+    assert d["triangles"].dtype == np.float64 and np.array_equal(d["triangles"], np.asarray(m.Triangles).reshape(-1, 3))
