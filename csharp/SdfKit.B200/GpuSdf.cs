@@ -3,7 +3,9 @@
 // `sdf.Target is GpuSdf` and take the native path; any other delegate (an opaque lambda, Sdfs.*, SdfFuncs.*) is
 // rejected with NotSupportedException -- there is no CPU fallback.  SOURCE ONLY (no .NET toolchain in this image).
 using System;
+using System.IO;
 using System.Numerics;
+using System.Runtime.ExceptionServices;
 using System.Runtime.InteropServices;
 using System.Text;
 
@@ -144,6 +146,32 @@ namespace SdfKit.B200
                     Native.Check(Native.sdfk_mesh_export(mesh, (float*)pv, (float*)pc, (float*)pn, pt, aabb));
                 return new Mesh(v, c, n, t);     // Mesh ctor re-measures Min/Max (Mesh.cs:21-28); aabb is equal
             } finally { Native.sdfk_mesh_destroy(mesh); }
+        }
+
+        /// Mesh.WriteObj (SdfKit/Mesh.cs:66-97): the OBJ text is formatted on the GPU and written to `stream` in chunks, byte for
+        /// byte what the reference's StreamWriter loop prints (float.ToString() text, 1-based indices, '\n' line ends).  An
+        /// exception thrown by the stream stops the native call and is rethrown here.
+        public static void WriteObj(Mesh mesh, Stream stream)
+        {
+            var ctx = GpuContext.Shared;
+            Exception? error = null;
+            var chunk = new byte[0];
+            Native.WriteFn sink = (bytes, n, _) => {
+                try {
+                    int len = checked((int)(ulong)n);
+                    if (chunk.Length < len) chunk = new byte[len];
+                    Marshal.Copy(bytes, chunk, 0, len);
+                    stream.Write(chunk, 0, len);
+                    return 0;
+                } catch (Exception e) { error = e; return 1; }
+            };
+            int status;
+            fixed (Vector3* pv = mesh.Vertices) fixed (Vector3* pn = mesh.Normals) fixed (int* pt = mesh.Triangles)
+                status = Native.sdfk_obj_write(ctx.Ptr, (float*)pv, mesh.Vertices.Length, (float*)pn, mesh.Normals.Length,
+                    pt, mesh.Triangles.Length, sink, IntPtr.Zero, out _);
+            GC.KeepAlive(sink);                // the delegate must outlive the native call that calls it
+            if (error is not null) ExceptionDispatchInfo.Capture(error).Throw();
+            Native.Check(status);
         }
 
         /// RayMarcher.Render (SdfKit/RayMarcher.cs:45-64): camera matrices from System.Numerics as in :95-108

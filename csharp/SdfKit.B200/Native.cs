@@ -12,6 +12,10 @@ namespace SdfKit.B200
         [UnmanagedFunctionPointer(CallingConvention.Cdecl)]
         public delegate void ProgressFn(float fraction, IntPtr user);
 
+        // sdfk_write_fn: one chunk of OBJ text in file order; 0 = continue, anything else stops sdfk_obj_write
+        [UnmanagedFunctionPointer(CallingConvention.Cdecl)]
+        public delegate int WriteFn(IntPtr bytes, UIntPtr n, IntPtr user);
+
         [DllImport(Lib)] public static extern IntPtr sdfk_last_error();
         [DllImport(Lib)] public static extern int sdfk_version();
 
@@ -47,12 +51,15 @@ namespace SdfKit.B200
         [DllImport(Lib)] public static extern int sdfk_ctx_set_option(IntPtr ctx, int option, int value);
         [DllImport(Lib)] public static extern int sdfk_ctx_store_bandwidth(IntPtr ctx, UIntPtr bytes, int reps, out double gbPerS);
         [DllImport(Lib)] public static extern int sdfk_mesh_destroy(IntPtr mesh);
+        // Mesh.WriteObj (Mesh.cs:66-97): the OBJ text formatted on the device, handed to `sink` chunk by chunk on the calling thread
+        [DllImport(Lib)] public static extern int sdfk_obj_write(IntPtr ctx, float* vertices, long nvertices, float* normals, long nnormals,
+            int* triangles, long nindices, WriteFn sink, IntPtr user, out long bytesWritten);
 
         // Not bound here (not needed by the drop-in; see include/sdfk.h): instrumentation (sdfk_ctx_mark / _elapsed / _timer_* /
         // _launch_count / _last_wall_ms / _stream / _create_on_stream, sdfk_mesh_stats, sdfk_sdf_check), the per-process slab API of
         // the torchrun path (sdfk_voxels_sample_slab / _sample_distances / _resample / _info / _layers / _part, sdfk_mesh_classify /
         // _emit / _emit_host / _device_ptrs / _part, sdfk_plan_layers, sdfk_render_device), pinned-buffer helpers (sdfk_host_alloc /
-        // _free) and the exhaustive self-tests (sdfk_constdiv_verify, sdfk_selftest_sqrt).
+        // _free) and the exhaustive self-tests (sdfk_constdiv_verify, sdfk_selftest_sqrt, sdfk_selftest_float_text).
         // Vec3Data.SaveTga / FloatData.SaveDepthTga payloads packed on the device (a quarter of the float image over PCIe):
         [DllImport(Lib)] public static extern int sdfk_render_bgr8(IntPtr ctx, IntPtr sdf, int w, int h, float* camPos, float* invViewProj,
             float near, float far, int iterations, int rowBegin, int rowEnd, byte* bgr);

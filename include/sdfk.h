@@ -200,6 +200,21 @@ int sdfk_mesh_part(sdfk_mesh* mesh, int part, sdfk_mesh** out, int64_t* vertex_b
 int sdfk_mesh_stats(sdfk_mesh* mesh, double stats[8]);
 int sdfk_mesh_destroy(sdfk_mesh* mesh);
 
+/* ---- Mesh.WriteObj (Mesh.cs:66-97) -----------------------------------------------------------------
+ * The OBJ text of host arrays -- "v x y z" per vertex, "vn x y z" per normal, "f a//a b//b c//c" per triangle (indices
+ * triangles[k] + 1 in 32-bit two's complement, as the reference's
+ * int arithmetic wraps), '\n' line ends, floats as .NET Core float.ToString() prints them -- formatted on device 0
+ * of the context and handed to `sink` in file order, in chunks, on the calling thread.  nnormals may differ from nvertices;
+ * nindices must be a multiple of 3; an empty mesh makes no sink call.  sink returns 0 to continue; anything else stops the
+ * call (SDFK_ERR_INVALID, the sink's value in the message).  The sink must not call into the same ctx.  bytes_written (may
+ * be NULL) receives the bytes the sink accepted.  The streams are idle again when the call returns, whatever the result. */
+typedef int (*sdfk_write_fn)(const void* bytes, size_t n, void* user);
+int sdfk_obj_write(sdfk_ctx* ctx, const float* vertices, int64_t nvertices, const float* normals, int64_t nnormals,
+                   const int32_t* triangles, int64_t nindices, sdfk_write_fn sink, void* user, int64_t* bytes_written);
+/* digests[i] = FNV-1a-64 of the .NET text (+ '\n') of every float with bit pattern in block first_block + i (2^20 each,
+ * in increasing order); first_block + nblocks <= 4096 */
+int sdfk_selftest_float_text(sdfk_ctx* ctx, uint32_t first_block, uint32_t nblocks, uint64_t* digests);
+
 /* ---- RayMarcher (RayMarcher.cs) ---------------------------------------------------------------------
  * cam_pos = translation of inverse(ViewTransform); inv_view_proj = inverse(ViewTransform * projection)
  * (RayMarcher.cs:95-108) -- computed by the caller.  rows [row_begin, row_end) of the w*h image are

@@ -10,6 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SDFK_LIB") or os.path.join(_HERE, "libsdfk.so")
 
 PROGRESS_FN = C.CFUNCTYPE(None, C.c_float, C.c_void_p)
+WRITE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_size_t, C.c_void_p)
 _fp = C.POINTER(C.c_float)
 _vp = C.c_void_p
 _i64p = C.POINTER(C.c_int64)
@@ -68,6 +69,8 @@ SIGNATURES = {
     "sdfk_mesh_part": (C.c_int, [_vp, C.c_int, C.POINTER(_vp), _i64p, _i64p]),
     "sdfk_mesh_stats": (C.c_int, [_vp, C.POINTER(C.c_double)]),
     "sdfk_mesh_destroy": (C.c_int, [_vp]),
+    "sdfk_obj_write": (C.c_int, [_vp, _fp, C.c_int64, _fp, C.c_int64, C.POINTER(C.c_int32), C.c_int64, WRITE_FN, _vp, _i64p]),
+    "sdfk_selftest_float_text": (C.c_int, [_vp, C.c_uint32, C.c_uint32, C.POINTER(C.c_uint64)]),
     "sdfk_render": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _fp, _fp, C.c_float, C.c_float, C.c_int, C.c_int, C.c_int, _fp]),
     "sdfk_render_depth": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _fp, _fp, C.c_float, C.c_int, C.c_int, C.c_int, _fp]),
     "sdfk_render_bgr8": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _fp, _fp, C.c_float, C.c_float, C.c_int, C.c_int, C.c_int,

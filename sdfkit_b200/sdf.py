@@ -95,7 +95,7 @@ class GpuSdf:
         N.check(N.lib().sdfk_sdf_to_mesh_host(self.ctx.handle, self.handle, N.fptr(vmin), N.fptr(vmax), int(nx), int(ny), int(nz),
                                               1 if clipToBounds else 0, float(isoValue), int(step), N.fptr(M), N.fptr(Nm), int(slabs),
                                               cb if progress else C.cast(None, N.PROGRESS_FN), None, C.byref(h)))
-        return GpuMesh(h).host_view()
+        return GpuMesh(h, self.ctx).host_view()
 
     def ToImage(self, width, height, *camera, verticalFieldOfViewDegrees=60.0, nearPlaneDistance=1.0,
                 farPlaneDistance=100.0, depthIterations=40, batchSize=SdfConfig.DefaultBatchSize,

@@ -4,6 +4,8 @@ The voxel field lives in HBM behind an sdfk_voxels handle (device layout x-faste
 arrays `Values[x,y,z]` / `Colors[x,y,z]` are materialised lazily, in the C# layout, on first access.
 """
 import ctypes as C
+import io
+import os
 
 import numpy as np
 
@@ -14,10 +16,12 @@ from . import numerics
 class Mesh:
     """SdfKit.Mesh (Mesh.cs): Vertices / Colors / Normals (n x 3 float32), Triangles (flat int32, 3 per triangle)."""
 
-    def __init__(self, vertices, colors, normals, triangles, vmin=None, vmax=None):
-        """Mesh(vertices, colors, normals, triangles) (Mesh.cs:21-28); Min/Max are measured unless the caller already has them."""
+    def __init__(self, vertices, colors, normals, triangles, vmin=None, vmax=None, ctx=None):
+        """Mesh(vertices, colors, normals, triangles) (Mesh.cs:21-28); Min/Max are measured unless the caller already has them.
+        ctx: the context that produced the mesh (None for a mesh built from host arrays); WriteObj formats on its GPU."""
         self.Vertices, self.Colors, self.Normals, self.Triangles = vertices, colors, normals, triangles
         self.Min, self.Max = vmin, vmax
+        self.ctx = ctx
         if vmin is None or vmax is None:
             self._measure()
 
@@ -63,7 +67,10 @@ class Mesh:
         return numerics.length3(self.Size) * np.float32(0.5)
 
     def WriteObj(self, path_or_file):
-        """Mesh.WriteObj (Mesh.cs:66-97): "v x y z", "vn x y z", "f i//i j//j k//k" (1-based)."""
+        """Mesh.WriteObj (Mesh.cs:66-97): "v x y z", "vn x y z", "f i//i j//j k//k" (1-based).  A mesh with a context is
+        formatted on its GPU (sdfk_obj_write), byte for byte the text of the host writer below, which serves the others."""
+        if self.ctx is not None:
+            return self._write_obj_device(path_or_file)
         fmt = _net_float
         close = False
         w = path_or_file
@@ -81,6 +88,37 @@ class Mesh:
         finally:
             if close:
                 w.close()
+
+    def _write_obj_device(self, path_or_file):
+        """Paths and binary files receive the chunks as they are (a memoryview over the page-locked stage, no copy); text
+        streams receive them decoded as ASCII.  An exception raised while writing (a full disk) stops the call and is
+        re-raised once the library has returned."""
+        v = N.f32c(self.Vertices).reshape(-1)
+        n = N.f32c(self.Normals).reshape(-1)
+        t = np.ascontiguousarray(self.Triangles, dtype=np.int32).reshape(-1)
+        close = isinstance(path_or_file, (str, os.PathLike))
+        f = open(path_or_file, "wb") if close else path_or_file
+        text = isinstance(f, io.TextIOBase)
+        errors = []
+
+        def sink(ptr, nbytes, _user):
+            try:
+                chunk = memoryview((C.c_ubyte * nbytes).from_address(ptr))
+                f.write(bytes(chunk).decode("ascii") if text else chunk)
+                return 0
+            except BaseException as e:          # noqa: B036 -- carried across the C frame and re-raised below
+                errors.append(e)
+                return 1
+        cb = N.WRITE_FN(sink)
+        try:
+            rc = N.lib().sdfk_obj_write(self.ctx.handle, N.fptr(v), len(v) // 3, N.fptr(n), len(n) // 3,
+                                        t.ctypes.data_as(C.POINTER(C.c_int32)), len(t), cb, None, None)
+        finally:
+            if close:
+                f.close()
+        if errors:
+            raise errors[0]
+        N.check(rc)
 
 
 def _net_float(x):
@@ -105,8 +143,9 @@ def _net_float(x):
 class GpuMesh:
     """Handle-level view of an sdfk_mesh (used by the multi-GPU driver and the benchmark)."""
 
-    def __init__(self, handle):
+    def __init__(self, handle, ctx=None):
         self.handle = handle
+        self.ctx = ctx                          # handed on to the host meshes made from this one
 
     def counts(self):
         nv, nt = C.c_int64(), C.c_int64()
@@ -130,7 +169,7 @@ class GpuMesh:
         aabb = np.zeros(6, dtype=np.float32)
         N.check(N.lib().sdfk_mesh_export(self.handle, N.fptr(v), N.fptr(c), N.fptr(n),
                                          t.ctypes.data_as(C.POINTER(C.c_int32)), N.fptr(aabb)))
-        return Mesh(v, c, n, t, aabb[:3].copy(), aabb[3:].copy())
+        return Mesh(v, c, n, t, aabb[:3].copy(), aabb[3:].copy(), ctx=self.ctx)
 
     def host_view(self):
         """Mesh over the page-locked host arrays of a mesh made by sdfk_sdf_to_mesh_host (zero copy).  The arrays keep
@@ -151,7 +190,7 @@ class GpuMesh:
         c = view(ptrs[1], nv, np.float32, (nv, 3))
         n = view(ptrs[2], nv, np.float32, (nv, 3))
         t = view(ptrs[3], nt, np.int32, (nt * 3,))
-        return Mesh(v, c, n, t, aabb[:3].copy(), aabb[3:].copy())
+        return Mesh(v, c, n, t, aabb[:3].copy(), aabb[3:].copy(), ctx=self.ctx)
 
     def destroy(self):
         if self.handle:
@@ -361,7 +400,7 @@ class MarchingCubes:
         h = C.c_void_p()
         N.check(N.lib().sdfk_mesh_create(volume.ctx.handle, volume.handle, float(isoValue), int(step), N.fptr(M), N.fptr(Nm),
                                          cb if progress else C.cast(None, N.PROGRESS_FN), None, C.byref(h)))
-        return GpuMesh(h)
+        return GpuMesh(h, volume.ctx)
 
     @staticmethod
     def CreateMesh(volume, isoValue=0.0, step=1, progress=None):
