@@ -157,12 +157,17 @@ int sdfk_voxels_destroy(sdfk_voxels* vox);
 
 /* ---- MarchingCubes.CreateMesh / Voxels.ToMesh (MarchingCubes.cs:39-92, Voxels.cs:67-70) -------------
  * transform / normal_transform: the matrices Mesh.Transform applies (MarchingCubes.cs:85-90, Mesh.cs:47-64),
- * computed by the caller; both NULL leaves the mesh in voxel-index space.                               */
+ * computed by the caller; both NULL leaves the mesh in voxel-index space.
+ * Any grid whose voxels fit in device memory is meshed: a grid with more cells or 128-cell chunks than one meshing job's
+ * 32-bit ids hold (from ~1626^3 on) is meshed in consecutive sub-slabs of cell layers, one after the other, into ONE mesh
+ * (the same arrays, handle and results as a one-job mesh).  The same holds per device on a multi-GPU context. */
 int sdfk_mesh_create(sdfk_ctx* ctx, sdfk_voxels* vox, float iso, int step, const float transform[16],
                      const float normal_transform[16], sdfk_progress_fn progress, void* user, sdfk_mesh** out);
 /* Slab meshing for multi-GPU jobs, in two phases around the caller's all-gather of counts:
  *   sdfk_mesh_classify: classify + scan the cell layers of this slab that lie in [k_begin, k_end) (global
  *                       cell-layer range this rank owns); reports how many vertices / triangles it owns.
+ *                       One call is one meshing job: fewer than 2^32 cells and 128-cell chunks in the classified layers
+ *                       (ghost layers included), else SDFK_ERR_UNSUPPORTED -- split the range over several calls.
  *   sdfk_mesh_emit:     write the owned vertices / triangles with global ids starting at vertex_base /
  *                       triangle_base (exclusive sums of the lower ranks' counts).                      */
 int sdfk_mesh_classify(sdfk_ctx* ctx, sdfk_voxels* vox, float iso, int step, int k_begin, int k_end,

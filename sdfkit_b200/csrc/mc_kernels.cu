@@ -17,6 +17,7 @@
 //   K4a mc_compact  active chunks -> one McRecord per active cell, in visiting order, + full per-chunk counts
 //   K4b mc_emit     per record: triangle indices, created vertices (position, colour), normals gathered
 //                   in the reference's accumulation order, -normalize, Mesh.Transform, AABB
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -1645,6 +1646,22 @@ cudaError_t mc_launch_emit(const McEmitParams& p, cudaStream_t s)
     const unsigned nv = p.vert_end - p.vert_begin;
     if (e != cudaSuccess || nv == 0) return e;
     mc_emit_verts_kernel<<<(nv + MC_VERT_PER_BLOCK - 1u) / MC_VERT_PER_BLOCK, MC_VERT_THREADS, 0, s>>>(p);
+    return cudaGetLastError();
+}
+
+__global__ void mc_offset_ids_kernel(int* __restrict__ ids, size_t n, int delta)
+{
+    for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (size_t)gridDim.x * blockDim.x) ids[k] += delta;
+}
+
+cudaError_t mc_launch_offset_ids(int* ids, size_t n, int delta, cudaStream_t s)
+{
+    if (n == 0 || delta == 0) return cudaSuccess;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const size_t blocks = std::min<size_t>((n + 255) / 256, (size_t)sms * 8);
+    mc_offset_ids_kernel<<<(unsigned)blocks, 256, 0, s>>>(ids, n, delta);
     return cudaGetLastError();
 }
 

@@ -96,5 +96,7 @@ cudaError_t mc_launch_boundary(const uint4* base, const uint4* abase, size_t idx
 // the same prefixes at the first chunk of each of nlayers cell layers (per_layer chunks apart): nlayers uint4 to mapped host memory
 cudaError_t mc_launch_layer_prefixes(const uint4* base, const uint4* abase, size_t per_layer, unsigned nlayers, void* dst_host_mapped, cudaStream_t s);
 cudaError_t mc_launch_emit(const McEmitParams& p, cudaStream_t s);
+// ids[k] += delta for k < n: the triangles of a mesh part emitted with vertex ids from 0 moved to its global vertex base
+cudaError_t mc_launch_offset_ids(int* ids, size_t n, int delta, cudaStream_t s);
 // nwords 32-bit words from device memory to MAPPED page-locked host memory, by a kernel (no copy engine involved)
 cudaError_t mc_launch_readback(const void* src_dev, void* dst_host_mapped, unsigned nwords, cudaStream_t s);
